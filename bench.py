@@ -8,6 +8,7 @@ L2O-DM (LSTM-20x2, identity preprocess) on separable Rastrigin, 1M coordinates P
 unroll T=100.  Synthetic data, random-init weights (seeded).
 
   python bench.py --gpus 1 --steps 5 --warmup 3
+  python bench.py --gpus 1 --steps 5 --warmup 3 --dump-outputs DIR   # + the last timed step's outputs as DIR/*.npy
   torchrun --nproc-per-node N ... bench.py --gpus N ...
   python bench.py --impl reference ...     # the CPU oracle (port of the reference's algorithm) on host cores
 """
@@ -49,7 +50,15 @@ def parse():
                     help="coordinates of the CPU-oracle sample (0 = best of the workload's default sample sizes)")
     ap.add_argument("--scaling", default="weak", choices=["weak", "strong"],
                     help="weak: --coords per GPU (default 1M each); strong: --coords in TOTAL (default 1M) sharded over the ranks")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed meta-step computed as DIR/<name>.npy "
+                         "(rank 0's view; under 64 MB in all) so that two builds can be compared output for output")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and (args.impl != "ours" or args.workload == "hrnn_convnet"):
+        ap.error("--dump-outputs covers the MetaOptimizer workloads of --impl ours")
+    return args
 
 
 # ------------------------------------------------------------------------------------------------
@@ -99,6 +108,34 @@ def make_problem(name, coords, rank, shard=None):
             "layers": (20, 20), "preprocess_name": "fc", "preprocess_options": {"dim": 20}, "scale": 0.01,
             "tanh_output": True}}}, "rnnprop"
     raise ValueError(name)
+
+
+DUMP_BYTES = 60 << 20   # array data of --dump-outputs; with the .npy headers the files stay under 64 MB
+
+
+def last_step_outputs(prog):
+    """What the last ``Session.run([fx, update, step])`` hands its caller: the objective over the unroll (``fx[T]`` is
+    the fetched fx), the optimizee's coordinates after the committed update and each net's weights after TF-Adam."""
+    out = {"fx": prog.last_fx.double(), "x": prog.X.float()}
+    for key, net in prog.nets.items():
+        out["theta_" + key] = net.theta.detach().float()
+    return {name: t.detach().cpu().numpy().reshape(-1) for name, t in out.items()}
+
+
+def dump_outputs(outdir, arrays):
+    """Write each array as ``outdir/<name>.npy``, DUMP_BYTES in all.  The smaller arrays are kept whole; one that does
+    not fit its share is cut to a seeded sample of its elements, the same indices in every run of the same size."""
+    os.makedirs(outdir, exist_ok=True)
+    import numpy as np
+    names = sorted(arrays, key=lambda k: arrays[k].nbytes)
+    left = DUMP_BYTES
+    for i, name in enumerate(names):
+        a = arrays[name]
+        cap = left // (len(names) - i) // a.itemsize
+        if a.size > cap:
+            a = a[np.sort(np.random.default_rng(0).choice(a.size, cap, replace=False))]
+        np.save(os.path.join(outdir, name + ".npy"), a)
+        left -= a.nbytes
 
 
 class ClockSampler(threading.Thread):
@@ -595,6 +632,8 @@ def main():
     launches = eng.launch_count() - l0
     t_dev = e0.elapsed_time(e1) / 1e3
     sampler.stop()
+    if args.dump_outputs and rank == 0:     # before the kernel timings and the e2e steps below overwrite them
+        dump_outputs(args.dump_outputs, last_step_outputs(prog))
     tt = torch.tensor([t_dev], dtype=torch.float64, device=dev)
     if distributed:
         dist.all_reduce(tt, op=dist.ReduceOp.MAX)
