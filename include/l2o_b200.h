@@ -312,6 +312,51 @@ int l2o_hrnn_coord_bwd(l2o_hrnn_handle h, const l2o_hrnn_bwd_args* a, void* stre
  * [6] raw update (fp32 [N]) */
 int l2o_hrnn_workspace_layout(l2o_hrnn_handle h, int64_t offsets[7]);
 
+/* ---------------------------------------------------------------------------------------------------------------
+ * Hand-written update rules: the two nets of the reference's factory that have no trainable variables.  A rule is one
+ * descriptor (no handle, nothing allocated); nothing differentiates through it (the optimizee gradient it consumes is
+ * stop-gradient'ed, DM/meta.py:322-329), so there is no backward entry point.
+ *
+ *   l2o_rule_state_floats   Sgd / Adam .initial_state_for_inputs                  DM/networks.py:370-371,415-420
+ *   l2o_rule_step           update, state' = net(g, state)  (+ x += update)       DM/networks.py:367-368,393-413, DM/meta.py:352-353
+ *   l2o_rule_unroll_fwd     the tf.while_loop body x T with such a net            DM/meta.py:338-376
+ *
+ * Arithmetic in fp32 with TF's order and roundings (Sgd: -lr*g ; Adam: t' = t+1, m' = b1*m + (1-b1)*g,
+ * v' = b2*v + (1-b2)*g^2, update = -lr*(m'/(1-b1^t')) / (sqrt(v'/(1-b2^t')) + eps)).  The hyper-parameters are
+ * doubles because the reference's are Python floats: (1 - b) is formed before the rounding to fp32.
+ * Adam state arena: [t, pad, pad, pad | m [n] | v [n]] (t is the fp32 step counter, DM/networks.py:404). */
+#define L2O_RULE_SGD 0   /* networks.Sgd    DM/networks.py:354-371 */
+#define L2O_RULE_ADAM 1  /* networks.Adam   DM/networks.py:374-420 */
+typedef struct {
+  int32_t kind;           /* L2O_RULE_* */
+  double learning_rate;   /* >= 0 */
+  double beta1, beta2;    /* Adam: in [0, 1) */
+  double epsilon;
+} l2o_rule_desc;
+typedef struct {
+  int64_t n;
+  const float* g;         /* [n] */
+  const float* state_in;  /* Adam: arena of n coordinates (t read on the device: CUDA-graph friendly) */
+  float* state_out;       /* Adam: must not overlap state_in */
+  float* x;               /* optional [n]: x += update */
+  float* delta;           /* optional [n]: the update */
+} l2o_rule_step_args;
+typedef struct {
+  int64_t n;
+  int32_t T;
+  int32_t opt_kind;       /* L2O_OPT_RASTRIGIN_SEP | L2O_OPT_QUADRATIC_DIAG (others: L2O_E_UNSUPPORTED) */
+  const float* opt_a;
+  const float* opt_b;
+  float opt_alpha;
+  float opt_fscale;
+  float* x;               /* [n] in/out: x_0 -> x_T */
+  float* state;           /* Adam: arena in/out (S_0 -> S_T) */
+  double* fx;             /* optional [T+1]: fx[t] += f(x_t) */
+} l2o_rule_unroll_args;
+int l2o_rule_state_floats(const l2o_rule_desc* d, int64_t n, int64_t* out); /* Sgd 0, Adam 4 + 2n */
+int l2o_rule_step(const l2o_rule_desc* d, const l2o_rule_step_args* a, void* stream);
+int l2o_rule_unroll_fwd(const l2o_rule_desc* d, const l2o_rule_unroll_args* a, void* stream);
+
 /* Number of this library's kernels launched so far in this process (bench.py's gpu_launches). */
 int64_t l2o_launch_count(void);
 const char* l2o_status_string(int status);

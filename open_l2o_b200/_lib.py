@@ -20,6 +20,7 @@ L2O_OK, L2O_E_INVALID, L2O_E_UNSUPPORTED, L2O_E_CUDA, L2O_E_NOMEM = 0, -1, -2, -
 PRE_IDENTITY, PRE_LOGSIGN, PRE_FC = 0, 1, 2
 OPT_NONE, OPT_RASTRIGIN_SEP, OPT_QUADRATIC_DIAG, OPT_QUADRATIC_BATCH = 0, 1, 2, 3
 ENGINE_AUTO, ENGINE_FFMA, ENGINE_TC = 0, 1, 2
+RULE_SGD, RULE_ADAM = 0, 1
 
 # every symbol include/l2o_b200.h declares (tests check the .so exports all of them)
 EXPORTS = [
@@ -32,6 +33,7 @@ EXPORTS = [
     "l2o_hrnn_workspace_bytes", "l2o_hrnn_init_state", "l2o_hrnn_prepare", "l2o_hrnn_step",
     "l2o_hrnn_set_global_sizes", "l2o_hrnn_reduce_layout", "l2o_hrnn_prepare_local", "l2o_hrnn_prepare_finish",
     "l2o_hrnn_step_local", "l2o_hrnn_step_finish", "l2o_hrnn_coord_bwd", "l2o_hrnn_workspace_layout",
+    "l2o_rule_state_floats", "l2o_rule_step", "l2o_rule_unroll_fwd",
 ]
 
 
@@ -93,6 +95,20 @@ class HrnnBwdArgs(C.Structure):
     _fields_ = [("theta", _fp), ("state_old", _fp), ("g", _fp), ("bias0", _fp), ("zero_flag", _fp), ("mean_log_lr", _fp),
                 ("d_state_new", _fp), ("d_upd", _fp), ("d_sums", _fp), ("d_state_old", _fp), ("d_theta", _fp),
                 ("d_bias0", _fp), ("d_mean_log_lr", _fp)]
+
+
+class RuleDesc(C.Structure):
+    _fields_ = [("kind", C.c_int32), ("learning_rate", C.c_double), ("beta1", C.c_double), ("beta2", C.c_double),
+                ("epsilon", C.c_double)]
+
+
+class RuleStepArgs(C.Structure):
+    _fields_ = [("n", C.c_int64), ("g", _fp), ("state_in", _fp), ("state_out", _fp), ("x", _fp), ("delta", _fp)]
+
+
+class RuleUnrollArgs(C.Structure):
+    _fields_ = [("n", C.c_int64), ("T", C.c_int32), ("opt_kind", C.c_int32), ("opt_a", _fp), ("opt_b", _fp),
+                ("opt_alpha", C.c_float), ("opt_fscale", C.c_float), ("x", _fp), ("state", _fp), ("fx", _fp)]
 
 
 class L2OError(RuntimeError):
@@ -223,6 +239,12 @@ def lib():
                  "l2o_hrnn_prepare_finish", "l2o_hrnn_step_local", "l2o_hrnn_step_finish"):
         getattr(L, name).argtypes = [C.c_void_p, C.POINTER(HrnnArgs), C.c_void_p]
         getattr(L, name).restype = C.c_int
+    L.l2o_rule_state_floats.argtypes = [C.POINTER(RuleDesc), C.c_int64, C.POINTER(C.c_int64)]
+    L.l2o_rule_state_floats.restype = C.c_int
+    L.l2o_rule_step.argtypes = [C.POINTER(RuleDesc), C.POINTER(RuleStepArgs), C.c_void_p]
+    L.l2o_rule_step.restype = C.c_int
+    L.l2o_rule_unroll_fwd.argtypes = [C.POINTER(RuleDesc), C.POINTER(RuleUnrollArgs), C.c_void_p]
+    L.l2o_rule_unroll_fwd.restype = C.c_int
     for name in ("l2o_status_string", "l2o_last_cuda_error", "l2o_version"):
         getattr(L, name).restype = C.c_char_p
     L.l2o_status_string.argtypes = [C.c_int]

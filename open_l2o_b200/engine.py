@@ -9,7 +9,8 @@ import torch
 
 from . import _lib
 from ._lib import (BwdArgs, NetDesc, StepArgs, UnrollArgs, L2OError, PRE_FC, PRE_IDENTITY, PRE_LOGSIGN,
-                   OPT_NONE, OPT_QUADRATIC_DIAG, OPT_RASTRIGIN_SEP, OPT_QUADRATIC_BATCH, ENGINE_AUTO, ENGINE_FFMA, ENGINE_TC)
+                   OPT_NONE, OPT_QUADRATIC_DIAG, OPT_RASTRIGIN_SEP, OPT_QUADRATIC_BATCH, ENGINE_AUTO, ENGINE_FFMA, ENGINE_TC,
+                   RULE_ADAM, RULE_SGD)
 
 _PRE = {"identity": PRE_IDENTITY, "LogAndSign": PRE_LOGSIGN, "fc": PRE_FC}
 OPT_KINDS = {"rastrigin_sep": OPT_RASTRIGIN_SEP, "quadratic_diag": OPT_QUADRATIC_DIAG,
@@ -237,6 +238,45 @@ class DenseNetHandle:
         a.n_total = n_total
         a.dtheta = _ptr(dtheta, torch.float64, "dtheta")
         _lib.check(_lib.lib().l2o_dense_unroll_bwd(self._h, C.byref(a), _stream()), "l2o_dense_unroll_bwd")
+
+
+class RuleHandle:
+    """A hand-written update rule (networks.Sgd / networks.Adam, DM/networks.py:354-420) on the ``l2o_rule_*``
+    kernels: state size, a fresh state, one step, a fused unroll.  No theta, no BPTT."""
+
+    n_in = 1
+
+    def __init__(self, kind: int, learning_rate: float, beta1: float = 0.9, beta2: float = 0.999,
+                 epsilon: float = 1e-8):
+        d = _lib.RuleDesc()
+        d.kind, d.learning_rate, d.beta1, d.beta2, d.epsilon = kind, learning_rate, beta1, beta2, epsilon
+        self.desc = d
+        self.state_size(0)   # validates the descriptor (negative rate, beta outside [0, 1), unknown kind)
+
+    def state_size(self, n: int) -> int:
+        """Floats of one state arena for n coordinates (Sgd 0, Adam 4 + 2n)."""
+        out = C.c_int64()
+        _lib.check(_lib.lib().l2o_rule_state_floats(C.byref(self.desc), n, C.byref(out)), "l2o_rule_state_floats")
+        return int(out.value)
+
+    def new_state(self, n: int, device) -> torch.Tensor:
+        return torch.zeros(max(self.state_size(n), 1), dtype=torch.float32, device=device)
+
+    def step(self, g, state_in, state_out, *, x=None, delta=None):
+        a = _lib.RuleStepArgs()
+        a.n = g.numel()
+        a.g = _ptr(g, name="g")
+        a.state_in, a.state_out = _ptr(state_in, name="state_in"), _ptr(state_out, name="state_out")
+        a.x, a.delta = _ptr(x, name="x"), _ptr(delta, name="delta")
+        _lib.check(_lib.lib().l2o_rule_step(C.byref(self.desc), C.byref(a), _stream()), "l2o_rule_step")
+
+    def unroll_fwd(self, n, T, state, *, opt_kind, opt_a, opt_b, opt_alpha=10.0, opt_fscale=1.0, x, fx=None):
+        a = _lib.RuleUnrollArgs()
+        a.n, a.T, a.opt_kind = n, T, opt_kind
+        a.opt_a, a.opt_b = _ptr(opt_a, name="opt_a"), _ptr(opt_b, name="opt_b")
+        a.opt_alpha, a.opt_fscale = opt_alpha, opt_fscale
+        a.x, a.state, a.fx = _ptr(x, name="x"), _ptr(state, name="state"), _ptr(fx, torch.float64, "fx")
+        _lib.check(_lib.lib().l2o_rule_unroll_fwd(C.byref(self.desc), C.byref(a), _stream()), "l2o_rule_unroll_fwd")
 
 
 def adam_step(theta, dtheta, m, v, k: int, lr=0.01, beta1=0.9, beta2=0.999, eps=1e-8):

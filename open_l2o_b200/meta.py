@@ -121,6 +121,11 @@ def _make_nets(variables, config, net_assignments):
     return nets, keys, subsets
 
 
+def _is_rule(net):
+    """Sgd / Adam: a hand-written rule, nothing to train and nothing to differentiate through."""
+    return isinstance(net, networks._Rule)
+
+
 class _Run(object):
     """A maximal contiguous slice of the flat coordinate arena served by one net."""
 
@@ -151,6 +156,14 @@ class _Program(object):
         print([c["name"] for c in self.constants])
         self.nets, self.net_keys, self.subsets = _make_nets(self.variables, optimizer._config, net_assignments)
         optimizer._nets = self.nets
+        if any(_is_rule(net) for net in self.nets.values()):
+            if optimizer.rnnprop:
+                raise NotImplementedError("Sgd / Adam nets in an RNNProp program: every net there is called as "
+                                          "net(m, g, state), which a hand-written rule does not take")
+            if optimizer.distributed:
+                raise NotImplementedError("Sgd / Adam nets in a sharded (_distributed=True) program")
+        # the nets with trainable variables: only they get a meta-gradient accumulator and meta-Adam slots
+        self.learned = {k: net for k, net in self.nets.items() if not _is_rule(net)}
 
         # flat arena: variables ordered so that each net's subset is contiguous where possible
         order = []
@@ -183,6 +196,8 @@ class _Program(object):
         one_net = len(self.runs) == 1 and self.runs[0].n == self.N
         if self.fused is not None and not (one_net and (len(self.variables) == 1 or self.fused.kind == "mlp_xent")):
             self.fused = None
+        if self.fused is not None and self.fused.kind == "quadratic_batch" and _is_rule(self.runs[0].net):
+            self.fused = None   # the rule unroll has no dense-group optimizee: step at a time instead
         # "producer" optimizees (SURVEY.md 8(f) row 4): f and df/dx come from ONE library kernel per step instead of
         # torch autograd (~15 launches); the unroll stays step-at-a-time (the gradient couples coordinates) and is
         # captured into one CUDA graph like every external-gradient unroll
@@ -190,9 +205,9 @@ class _Program(object):
         if self.fused is not None and self.fused.kind in _PRODUCER_KINDS:
             self.producer, self.fused = self.fused, None
         self.adam = {k: dict(m=torch.zeros_like(net.theta), v=torch.zeros_like(net.theta), k=0)
-                     for k, net in self.nets.items()}
+                     for k, net in self.learned.items()}
         self.dtheta = {k: torch.zeros(net.theta.numel(), dtype=torch.float64, device=self.device)
-                       for k, net in self.nets.items()}
+                       for k, net in self.learned.items()}
         self.step_placeholder = Placeholder("step")
         # per-variable scale placeholders (random-scaling trick, DM/meta_dm_train.py:336-338,384-385): fx = f(x * scale)
         self.scale_placeholders = [Placeholder(v["name"] + "_scale") for v in self.variables]
@@ -210,6 +225,12 @@ class _Program(object):
         T = self.T
         for r in self.runs:
             r.state = r.net.handle.new_state(r.n, self.device)
+            r.rule = _is_rule(r.net)
+            if r.rule:
+                # no checkpoints, no recorded gradients, no BPTT scratch: the state ping-pongs between two arenas
+                r.pp = (r.net.handle.new_state(r.n, self.device), r.net.handle.new_state(r.n, self.device))
+                r.x_work = torch.zeros(r.n, device=self.device)
+                continue
             r.ckpt = torch.zeros((T + 1) * max(r.net.handle.state_size(r.n), 1), device=self.device)
             r.g_rec = torch.zeros(T + 1, r.n, device=self.device)
             r.x_work = torch.zeros(r.n, device=self.device)
@@ -353,6 +374,14 @@ class _Program(object):
         r, T, f = self.runs[0], self.T, self.fused
         h = r.net.handle
         r.x_work.copy_(self.X)
+        if r.rule:
+            r.pp[0].copy_(r.state)
+            self.fx_buf.zero_()
+            h.unroll_fwd(r.n, T, r.pp[0], opt_kind=_engine.OPT_KINDS[f.kind],
+                         opt_a=self.const_vals[f.a].reshape(-1), opt_b=self.const_vals[f.b].reshape(-1),
+                         opt_alpha=f.alpha, opt_fscale=f.fscale, x=r.x_work, fx=self.fx_buf)
+            r.state_final = r.pp[0]
+            return self.fx_buf
         state = r.ckpt[:max(h.state_size(r.n), 1)]
         work_state = r.state.clone()
         self.fx_buf.zero_()
@@ -377,6 +406,9 @@ class _Program(object):
         Xw = self.X.clone()
         fxs = []
         for r in self.runs:
+            if r.rule:
+                r.pp[0].copy_(r.state)
+                continue
             r.ckpt[:max(r.net.handle.state_size(r.n), 1)].copy_(r.state)
             if r.net.handle.n_in == 2:
                 r.m_work.copy_(r.m)
@@ -386,6 +418,9 @@ class _Program(object):
             fxs.append(fx)
             for r in self.runs:
                 h = r.net.handle
+                if r.rule:
+                    h.step(g[r.off:r.off + r.n], r.pp[t % 2], r.pp[(t + 1) % 2], x=Xw[r.off:r.off + r.n])
+                    continue
                 slot = max(h.state_size(r.n), 1)
                 r.g_rec[t].copy_(g[r.off:r.off + r.n])
                 kw = {}
@@ -401,7 +436,8 @@ class _Program(object):
         if train:
             fx, g = self._value_and_grad(Xw)
             for r in self.runs:
-                r.g_rec[T].copy_(g[r.off:r.off + r.n])
+                if not r.rule:
+                    r.g_rec[T].copy_(g[r.off:r.off + r.n])
         else:
             if self.producer is not None:
                 fx = self._produce(Xw)[0]
@@ -410,8 +446,11 @@ class _Program(object):
                     fx = self._loss_at(Xw)
         fxs.append(fx)
         for r in self.runs:
-            slot = max(r.net.handle.state_size(r.n), 1)
-            r.state_final = r.ckpt[T * slot:(T + 1) * slot]
+            if r.rule:
+                r.state_final = r.pp[T % 2]
+            else:
+                slot = max(r.net.handle.state_size(r.n), 1)
+                r.state_final = r.ckpt[T * slot:(T + 1) * slot]
             r.x_work = Xw[r.off:r.off + r.n]
         self._Xw = Xw
         return torch.stack([f.reshape(()).double() for f in fxs])
@@ -424,6 +463,8 @@ class _Program(object):
             for d in self.dtheta.values():
                 d.zero_()
             for r in self.runs:
+                if r.rule:
+                    continue
                 h = r.net.handle
                 in_seq = r.feat_rec if h.n_in == 2 else r.g_rec
                 h.unroll_bwd(r.net.theta, r.n, self.T, in_seq, r.ckpt, self.dtheta[r.key], g_rec=r.g_rec,
@@ -509,6 +550,8 @@ class _Program(object):
                 for d in self.dtheta.values():
                     d.zero_()
                 for r in self.runs:
+                    if r.rule:
+                        continue
                     h = r.net.handle
                     in_seq = r.feat_rec if h.n_in == 2 else r.g_rec
                     h.unroll_bwd(r.net.theta, r.n, T, in_seq, r.ckpt, self.dtheta[r.key], g_rec=r.g_rec,
@@ -534,7 +577,7 @@ class _Program(object):
                         .reshape(v["shape"]).cpu().numpy() for j, v in enumerate(self.variables)]
         self.last_fx = fx
         if train:
-            for k, net in self.nets.items():
+            for k, net in self.learned.items():
                 ad = self.adam[k]
                 ad["k"] += 1
                 _engine.adam_step(net.theta, self.dtheta[k], ad["m"], ad["v"], ad["k"], lr=self.learning_rate)
@@ -564,6 +607,8 @@ class _MtTask(object):
     def __init__(self, prog, index):
         self.prog, self.index = prog, index
         T = prog.T
+        if len(prog.learned) != len(prog.nets):
+            raise NotImplementedError("imitation tasks with an Sgd / Adam net (nothing to imitate with)")
         self.subsets = []
         for key, subset in zip(prog.net_keys, prog.subsets):
             runs = [r for r in prog.runs if r.key == key]
@@ -655,6 +700,7 @@ class MetaOptimizer(object):
 
     beta1 = 0.95
     beta2 = 0.95
+    rnnprop = False   # RNNProp programs call every net as net(m, g, state)
 
     def __init__(self, **kwargs):
         """``MetaOptimizer(**net_config)`` exactly as the reference (DM/meta.py:228): every keyword is a net id.  The
@@ -715,11 +761,20 @@ class MetaOptimizer(object):
         """Returns ops minimizing the meta-loss with Adam (DM/meta.py:398-414)."""
         info = self.meta_loss(make_loss, len_unroll, **kwargs)
         self.program.learning_rate = learning_rate
+        self._check_trainable()
         return MetaStep(Op("step", self.program), *info[1:])
+
+    def _check_trainable(self):
+        """tf.train.AdamOptimizer.minimize raises when no net has a variable (Sgd / Adam only): the optimizee and
+        state variables are trainable=False (DM/meta.py:60-77,115-120)."""
+        if not self.program.learned:
+            raise ValueError("No variables to optimize: every net of this meta-optimizer is a hand-written rule")
 
 
 class RNNpropMetaOptimizer(MetaOptimizer):
     """DM/meta_rnnprop_train.py / meta_rnnprop_eval.py: per-coordinate Adam moments feed the net."""
+
+    rnnprop = True
 
     def __init__(self, beta1=0.95, beta2=0.95, **kwargs):
         super(RNNpropMetaOptimizer, self).__init__(**kwargs)

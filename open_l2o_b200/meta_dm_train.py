@@ -53,6 +53,7 @@ class MetaOptimizer(_meta.MetaOptimizer):
         """DM/meta_dm_train.py:529-558."""
         info = _meta.MetaOptimizer.meta_loss(self, make_loss, len_unroll, **kwargs)
         self.program.learning_rate = learning_rate
+        self._check_trainable()
         extras = self._extras(self.program)
         return (MetaStep(Op("step", self.program), *info[1:]),) + extras
 

@@ -12,6 +12,8 @@ from .meta_dm_train import VariableRef
 
 
 class MetaOptimizer(_meta.MetaOptimizer):
+    rnnprop = True
+
     def __init__(self, beta1, beta2, **kwargs):
         """DM/meta_rnnprop_eval.py:230-256."""
         super(MetaOptimizer, self).__init__(**kwargs)

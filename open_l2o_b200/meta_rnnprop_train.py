@@ -15,6 +15,8 @@ from .meta import MetaLoss, MetaStep, Op, Session  # noqa: F401  (re-exported li
 
 
 class MetaOptimizer(_dm.MetaOptimizer):
+    rnnprop = True
+
     def __init__(self, num_mt, beta1, beta2, **kwargs):
         """DM/meta_rnnprop_train.py:230-257."""
         super(MetaOptimizer, self).__init__(num_mt, **kwargs)

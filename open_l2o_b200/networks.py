@@ -313,11 +313,73 @@ class KernelDeepLSTM(Network):
         return delta.reshape(inputs.shape), st
 
 
-class Sgd(Network):
-    def __init__(self, *a, **k):
-        raise NotImplementedError("Sgd baseline net is outside the accelerated hot path (SURVEY.md section 2)")
+class _Rule(Network):
+    """A hand-written update rule: no trainable variables, no theta; the step runs in ``l2o_rule_step``."""
+
+    def variable_shapes(self):
+        return []
+
+    def get_variables(self):
+        return []
+
+    def set_variables(self, data):
+        pass
+
+    @property
+    def handle(self):
+        return self._handle
+
+    def _step(self, g, arena_in=None):
+        flat = g.reshape(-1).contiguous()
+        arena_out = torch.empty_like(arena_in) if arena_in is not None else None
+        delta = torch.empty_like(flat)
+        self._handle.step(flat, arena_in, arena_out, delta=delta)
+        return delta.reshape(g.shape), arena_out
 
 
-class Adam(Network):
-    def __init__(self, *a, **k):
-        raise NotImplementedError("Adam baseline net is outside the accelerated hot path (SURVEY.md section 2)")
+class Sgd(_Rule):
+    """Identity network which acts like SGD: update = -learning_rate * g (DM/networks.py:354-371)."""
+
+    def __init__(self, learning_rate=0.001, name="sgd"):
+        self.name = name
+        self._learning_rate = learning_rate
+        self._handle = _engine.RuleHandle(_engine.RULE_SGD, learning_rate)
+
+    def __call__(self, inputs, prev_state):
+        return self._step(inputs)[0], []
+
+    def initial_state_for_inputs(self, inputs, **kwargs):
+        return []
+
+
+class Adam(_Rule):
+    """Adam as an optimizer net (DM/networks.py:374-420).  State (t, m, v): a 0-d step counter and [N, 1] moments,
+    views of one arena [t, pad, pad, pad | m | v] (include/l2o_b200.h)."""
+
+    def __init__(self, learning_rate=1e-3, beta1=0.9, beta2=0.999, epsilon=1e-8, name="adam"):
+        self.name = name
+        self._learning_rate, self._beta1, self._beta2, self._epsilon = learning_rate, beta1, beta2, epsilon
+        self._handle = _engine.RuleHandle(_engine.RULE_ADAM, learning_rate, beta1, beta2, epsilon)
+
+    @staticmethod
+    def state_views(arena, n):
+        return arena[0], arena[4:4 + n].view(n, 1), arena[4 + n:4 + 2 * n].view(n, 1)
+
+    def _wrap_state(self, arena, n):
+        st = State(self.state_views(arena, n))
+        st.arena = arena
+        return st
+
+    def __call__(self, g, prev_state):
+        n = g.numel()
+        arena = getattr(prev_state, "arena", None)
+        if arena is None:
+            t, m, v = prev_state
+            arena = torch.cat([t.reshape(1).float(), torch.zeros(3, device=g.device), m.reshape(-1).float(),
+                               v.reshape(-1).float()]).contiguous()
+        update, arena_out = self._step(g, arena)
+        return update, self._wrap_state(arena_out, n)
+
+    def initial_state_for_inputs(self, inputs, **kwargs):
+        n = int(np.prod(inputs.shape)) if len(inputs.shape) else 1
+        return self._wrap_state(self._handle.new_state(n, inputs.device), n)

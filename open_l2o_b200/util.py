@@ -89,6 +89,14 @@ def get_config(problem_name, path=None, mode=None, num_hidden_layer=None, net_na
         problem = problems.simple()
         net_config = {"cw": {"net": "CoordinateWiseDeepLSTM", "net_options": {"layers": (), "initializer": "zeros"},
                              "net_path": path}}
+    elif problem_name == "simple-multi":
+        problem = problems.simple_multi_optimizer()
+        net_config = {
+            "cw": {"net": "CoordinateWiseDeepLSTM", "net_options": {"layers": (), "initializer": "zeros"},
+                   "net_path": path},
+            "adam": {"net": "Adam", "net_options": {"learning_rate": 0.01}},
+        }
+        net_assignments = [("cw", ["x_0"]), ("adam", ["x_1"])]
     elif problem_name == "quadratic":
         problem = problems.quadratic(batch_size=128, num_dims=10)
         net_config = _cw20(path)
